@@ -1,7 +1,8 @@
 """-m gpu parity tests: the CUDA path (through the C ABI) against the oracle, bit for bit.
 
 Oracle = oracle/_ref/libaisref.so (the unmodified reference, strict IEEE flags) when it was built, else the
-pinned C restatement oracle/libaisoracle.so.  Integer/byte outputs (frames, NMEA) and -- because every kernel
+pinned C restatement oracle/libaisoracle.so; where the C restatement does not cover a case (-go DSK / FP_DS, the V2 and
+Challenger models), the reference's results stored in tests/golden/ref_results.json.  Integer/byte outputs (frames, NMEA) and -- because every kernel
 replays the reference's operation order -- all float taps are required to be BIT-IDENTICAL (tolerance 0);
 the north_star tolerance for floats (1e-5 rel) is therefore met with margin.
 """
@@ -10,6 +11,7 @@ import pytest
 
 import aisgpu
 import aissynth as S
+import golden_util as G
 import oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -33,6 +35,20 @@ def first_diff(a, b):
     return (int(d[0]), int(len(d))) if len(d) else (-1, 0)
 
 
+def tap_table(model):
+    """(name, engine tap, oracle tap) for every tap compared per stream and channel."""
+    t = [("C", lambda e, s, ch: e.tap(aisgpu.TAP_C, s, ch), lambda r, ch: r.tap_c(O.TAP_CA + ch))]
+    if model == aisgpu.MODEL_DEFAULT:
+        t += [("CGF", lambda e, s, ch: e.tap(aisgpu.TAP_CGF, s, ch), lambda r, ch: r.tap_c(O.TAP_CGF_A + ch)),
+              ("FIR17", lambda e, s, ch: e.tap(aisgpu.TAP_FIR, s, ch), lambda r, ch: r.tap_c(O.TAP_FC_A + ch))]
+    else:
+        t += [("FM", lambda e, s, ch: e.tap(aisgpu.TAP_FM, s, ch, dtype=np.float32), lambda r, ch: r.tap_f(O.TAP_FM_A + ch)),
+              ("FIR37", lambda e, s, ch: e.tap(aisgpu.TAP_FIR, s, ch, dtype=np.float32), lambda r, ch: r.tap_f(O.TAP_FR_A + ch))]
+    for ph in range(1 if model == aisgpu.MODEL_BASE else 5):
+        t.append(("DEC%d" % ph, lambda e, s, ch, ph=ph: e.tap(aisgpu.TAP_DEC, s, ch + 2 * ph, dtype=np.float32), lambda r, ch, ph=ph: r.tap_f(ch * 5 + ph)))
+    return t
+
+
 def run_case(built, model, fs, N, nchunks, B, ps_ema=True, afc_wide=True, droop=True, fmt=aisgpu.FMT_CF32, check_taps=True, seed0=0, dsk=False,
              fp_ds=False):
     xs = [S.random_stream(fs, N * nchunks, seed0 + s)[0] for s in range(B)]
@@ -54,71 +70,46 @@ def run_case(built, model, fs, N, nchunks, B, ps_ema=True, afc_wide=True, droop=
         per = 1
     flags = (O.FLAG_PS_EMA if ps_ema else 0) | (O.FLAG_AFC_WIDE if afc_wide else 0) | (O.FLAG_DROOP if droop else 0)
     flags |= (O.FLAG_DSK if dsk else 0) | (O.FLAG_FP_DS if fp_ds else 0)
-    if (dsk or fp_ds) and not O.have_ref():
-        pytest.skip("-go DSK / FP_DS are checked against the compiled reference only")
+    taps = tap_table(model) if check_taps else []
+
+    def oracle_side(Model):
+        """Digests of every tap (per stream, channel; per-submit block lengths included) and of every stream's messages."""
+        refs = [Model(model=model, sample_rate=fs, fmt=fmt, flags=flags, taps=True) for _ in range(B)]
+        d = {"%s %d %d" % (t[0], s, ch): G.Digest() for t in taps for s in range(B) for ch in range(2)}
+        msgs = [[] for _ in range(B)]
+        for c in range(nchunks):
+            for s in range(B):
+                refs[s].push(raw[s][c * N * per:(c + 1) * N * per])
+                for ch in range(2):
+                    for name, _, ref_tap in taps:
+                        d["%s %d %d" % (name, s, ch)].add(ref_tap(refs[s], ch))
+                msgs[s] += refs[s].messages()
+        return {"taps": {k: v.value() for k, v in d.items()}, "messages": [G.msgs_digest(m) for m in msgs]}
+
+    if dsk or fp_ds:  # the C port has no -go DSK / FP_DS: the reference, or its stored digests
+        want = G.reference("parity %r" % ((model, fs, N, nchunks, B, ps_ema, afc_wide, droop, fmt, check_taps, seed0, dsk, fp_ds),),
+                           lambda: oracle_side(O.RefModel))
+    else:
+        want = oracle_side(oracle_model)
     eng = aisgpu.Engine(model=model, sample_rate=fs, fmt=fmt, n_streams=B, max_chunk=N, ps_ema=ps_ema, afc_wide=afc_wide,
                         droop=droop, taps=check_taps, dsk=dsk, fp_ds=fp_ds)
-    refs = [oracle_model(model=model, sample_rate=fs, fmt=fmt, flags=flags, taps=True) for _ in range(B)]
-    problems = []
+    d = {k: G.Digest() for k in want["taps"]}
     got_msgs = [[] for _ in range(B)]
-    want_msgs = [[] for _ in range(B)]
     for c in range(nchunks):
         batch = np.stack([r[c * N * per:(c + 1) * N * per] for r in raw])
         eng.submit(batch, N)
         for s in range(B):
-            refs[s].push(raw[s][c * N * per:(c + 1) * N * per])
-        if check_taps:
-            for s in range(B):
-                for ch in range(2):
-                    want = refs[s].tap_c(O.TAP_CA + ch)
-                    got = eng.tap(aisgpu.TAP_C, s, ch)
-                    if not bits_equal(got, want):
-                        problems.append(("C", c, s, ch, len(got), len(want)) + first_diff(got, want))
-                    if model == aisgpu.MODEL_DEFAULT:
-                        want = refs[s].tap_c(O.TAP_CGF_A + ch)
-                        got = eng.tap(aisgpu.TAP_CGF, s, ch)
-                        if not bits_equal(got, want):
-                            problems.append(("CGF", c, s, ch, len(got), len(want)) + first_diff(got, want))
-                        want = refs[s].tap_c(O.TAP_FC_A + ch)
-                        got = eng.tap(aisgpu.TAP_FIR, s, ch)
-                        if not bits_equal(got, want):
-                            problems.append(("FIR17", c, s, ch, len(got), len(want)) + first_diff(got, want))
-                    else:
-                        want = refs[s].tap_f(O.TAP_FM_A + ch)
-                        got = eng.tap(aisgpu.TAP_FM, s, ch, dtype=np.float32)
-                        if not bits_equal(got, want):
-                            problems.append(("FM", c, s, ch, len(got), len(want)) + first_diff(got, want))
-                        want = refs[s].tap_f(O.TAP_FR_A + ch)
-                        got = eng.tap(aisgpu.TAP_FIR, s, ch, dtype=np.float32)
-                        if not bits_equal(got, want):
-                            problems.append(("FIR37", c, s, ch, len(got), len(want)) + first_diff(got, want))
-                    nph = 1 if model == aisgpu.MODEL_BASE else 5
-                    for ph in range(nph):
-                        want = refs[s].tap_f(ch * 5 + ph)
-                        got = eng.tap(aisgpu.TAP_DEC, s, ch + 2 * ph, dtype=np.float32)
-                        if not bits_equal(got, want):
-                            problems.append(("DEC", c, s, ch, ph, len(got), len(want)) + first_diff(got, want))
-            if c == 0:
-                rot_w = None  # the oracle does not expose the phasor; C taps cover it
+            for ch in range(2):
+                for name, eng_tap, _ in taps:
+                    d["%s %d %d" % (name, s, ch)].add(eng_tap(eng, s, ch))
         for m in eng.poll():
             got_msgs[m.stream].append(m)
-        for s in range(B):
-            want_msgs[s] += refs[s].messages()
-    nmsg = 0
-    for s in range(B):
-        g = [(m.key(), m.start_idx, m.end_idx) for m in got_msgs[s]]
-        w = [(m.key(), m.start_idx, m.end_idx) for m in want_msgs[s]]
-        nmsg += len(w)
-        if g != w:
-            problems.append(("MSG", s, len(g), len(w), [x for x in g if x not in w][:2], [x for x in w if x not in g][:2]))
-        else:
-            for a, b in zip(got_msgs[s], want_msgs[s]):
-                if np.float32(a.level).view(np.uint32) != np.float32(b.level).view(np.uint32) or \
-                        np.float32(a.ppm).view(np.uint32) != np.float32(b.ppm).view(np.uint32):
-                    problems.append(("TAG", s, a.level, b.level, a.ppm, b.ppm))
     eng.close()
+    # taps bit for bit; messages (key, start/end idx) and tags (level, ppm bit patterns) in order, per stream
+    problems = [(k, d[k].value()[0], want["taps"][k][0]) for k in d if d[k].value() != want["taps"][k]]
+    problems += [("MSG", s, len(got_msgs[s]), want["messages"][s][0]) for s in range(B) if G.msgs_digest(got_msgs[s]) != want["messages"][s]]
     assert not problems, "parity problems (first 12): %r" % (problems[:12],)
-    return nmsg
+    return sum(w[0] for w in want["messages"])
 
 
 def test_default_1536k(built):
@@ -249,7 +240,7 @@ def test_dsk_buckets(built, fs, N, model):
     # DownsampleKFilter /3, exact and interpolated (CIC -> Upsample -> /3); rates outside those buckets keep their chain
     n = run_case(built, model, fs, N, 6, 2, check_taps=False, seed0=51, dsk=True)
     assert n >= 2
-    if fs != 1536000:
+    if fs != 1536000 and O.have_ref():
         resampler_taps(fs, N, 6, model, dsk=True)
 
 
@@ -277,51 +268,49 @@ def test_fp_ds_needs_cu8(built):
 
 
 def run_v2_case(fs, N, nchunks, B, check_taps, seed0, fmt=aisgpu.FMT_CF32):
-    """Model 11 "v2_base" (reference DSP/Decoder/V2/V2Engine.cpp, Model.cpp:440-460) against the compiled reference."""
-    if not O.have_ref():
-        pytest.skip("the V2 engine is checked against the compiled reference only")
+    """Model 11 "v2_base" (reference DSP/Decoder/V2/V2Engine.cpp, Model.cpp:440-460) against the compiled reference
+    (its stored digests where oracle/_ref was not built)."""
     xs = [S.random_stream(fs, N * nchunks, seed0 + s, bursts_per_sec=(6, 12))[0] for s in range(B)]
     per = 1
     if fmt == aisgpu.FMT_CU8:
         xs = [S.to_cu8(x) for x in xs]
         per = 2
     N_el = N * per  # array elements per chunk
+    names = ("V2.CGF", "V2.FIR17", "V2.FIR37")
+
+    def reference():
+        refs = [O.RefModel(model=O.MODEL_V2, sample_rate=fs, fmt=fmt, taps=check_taps) for _ in range(B)]
+        taps = {"%s %d %d" % (n, s, ch): G.Digest() for n in names for s in range(B) for ch in range(2)}
+        want = [[] for _ in range(B)]
+        for c in range(nchunks):
+            for s in range(B):
+                refs[s].push(xs[s][c * N_el:(c + 1) * N_el])
+                if check_taps:
+                    for ch in range(2):
+                        for n, w in zip(names, (refs[s].tap_c(O.TAP_CGF_A + ch), refs[s].tap_c(O.TAP_FC_A + ch), refs[s].tap_f(O.TAP_FR_A + ch))):
+                            taps["%s %d %d" % (n, s, ch)].add(w)
+                want[s] += refs[s].messages()
+        return {"taps": {k: d.value() for k, d in taps.items()} if check_taps else {}, "messages": [G.msgs_digest(w) for w in want]}
+
+    want = G.reference("v2 %r" % ((fs, N, nchunks, B, check_taps, seed0, fmt),), reference)
     eng = aisgpu.Engine(model=aisgpu.MODEL_V2, sample_rate=fs, fmt=fmt, n_streams=B, max_chunk=N, taps=check_taps)
-    refs = [O.RefModel(model=O.MODEL_V2, sample_rate=fs, fmt=fmt, taps=check_taps) for _ in range(B)]
-    problems = []
+    taps = {k: G.Digest() for k in want["taps"]}
     got = [[] for _ in range(B)]
-    want = [[] for _ in range(B)]
     for c in range(nchunks):
         eng.submit(np.stack([x[c * N_el:(c + 1) * N_el] for x in xs]), N)
-        for s in range(B):
-            refs[s].push(xs[s][c * N_el:(c + 1) * N_el])
         if check_taps:
             for s in range(B):
                 for ch in range(2):
-                    for name, g, w in (("V2.CGF", eng.tap(aisgpu.TAP_CGF, s, ch), refs[s].tap_c(O.TAP_CGF_A + ch)),
-                                       ("V2.FIR17", eng.tap(aisgpu.TAP_FIR, s, ch), refs[s].tap_c(O.TAP_FC_A + ch)),
-                                       ("V2.FIR37", eng.tap(aisgpu.TAP_FM, s, ch, dtype=np.float32), refs[s].tap_f(O.TAP_FR_A + ch))):
-                        if not bits_equal(g, w):
-                            problems.append((name, c, s, ch, len(g), len(w)) + first_diff(g, w))
+                    for n, g in zip(names, (eng.tap(aisgpu.TAP_CGF, s, ch), eng.tap(aisgpu.TAP_FIR, s, ch), eng.tap(aisgpu.TAP_FM, s, ch, dtype=np.float32))):
+                        taps["%s %d %d" % (n, s, ch)].add(g)
         for m in eng.poll():
             got[m.stream].append(m)
-        for s in range(B):
-            want[s] += refs[s].messages()
-    n = 0
-    for s in range(B):
-        g = [(m.key(), m.start_idx, m.end_idx) for m in got[s]]
-        w = [(m.key(), m.start_idx, m.end_idx) for m in want[s]]
-        n += len(w)
-        if g != w:
-            problems.append(("MSG", s, len(g), len(w), [x for x in g if x not in w][:2], [x for x in w if x not in g][:2]))
-        else:
-            for a, b in zip(got[s], want[s]):
-                if np.float32(a.level).view(np.uint32) != np.float32(b.level).view(np.uint32) or \
-                        np.float32(a.ppm).view(np.uint32) != np.float32(b.ppm).view(np.uint32):
-                    problems.append(("TAG", s, a.level, b.level, a.ppm, b.ppm))
     eng.close()
+    # every block's taps bit for bit; messages (key, start/end idx) and tags (level, ppm bit patterns) in order, per stream
+    problems = [k for k in taps if taps[k].value() != want["taps"][k]]
+    problems += [("MSG", s, len(got[s]), want["messages"][s][0]) for s in range(B) if G.msgs_digest(got[s]) != want["messages"][s]]
     assert not problems, "parity problems (first 12): %r" % (problems[:12],)
-    return n
+    return sum(w[0] for w in want["messages"])
 
 
 def test_v2_engine_blockwise_taps(built):
@@ -343,37 +332,31 @@ def test_v2_engine_cu8(built):
 
 
 def run_msg_case(model, fs, N, nchunks, B, seed0, fmt=aisgpu.FMT_CF32, bursts=(6, 12)):
-    """Frames + tags of a model the oracle has no taps for, against the compiled reference."""
-    if not O.have_ref():
-        pytest.skip("checked against the compiled reference only")
+    """Frames + tags of a model the oracle has no taps for, against the compiled reference (its stored digests where
+    oracle/_ref was not built)."""
     xs = [S.random_stream(fs, N * nchunks, seed0 + s, bursts_per_sec=bursts)[0] for s in range(B)]
+
+    def reference():
+        refs = [O.RefModel(model=model, sample_rate=fs, fmt=fmt) for _ in range(B)]
+        want = [[] for _ in range(B)]
+        for c in range(nchunks):
+            for s in range(B):
+                refs[s].push(xs[s][c * N:(c + 1) * N])
+                want[s] += refs[s].messages()
+        return [G.msgs_digest(w) for w in want]
+
+    want = G.reference("msgs %r" % ((model, fs, N, nchunks, B, seed0, fmt, bursts),), reference)
     eng = aisgpu.Engine(model=model, sample_rate=fs, fmt=fmt, n_streams=B, max_chunk=N)
-    refs = [O.RefModel(model=model, sample_rate=fs, fmt=fmt) for _ in range(B)]
     got = [[] for _ in range(B)]
-    want = [[] for _ in range(B)]
     for c in range(nchunks):
         eng.submit(np.stack([x[c * N:(c + 1) * N] for x in xs]), N)
-        for s in range(B):
-            refs[s].push(xs[s][c * N:(c + 1) * N])
         for m in eng.poll():
             got[m.stream].append(m)
-        for s in range(B):
-            want[s] += refs[s].messages()
-    problems, n = [], 0
-    for s in range(B):
-        g = [(m.key(), m.start_idx, m.end_idx) for m in got[s]]
-        w = [(m.key(), m.start_idx, m.end_idx) for m in want[s]]
-        n += len(w)
-        if g != w:
-            problems.append(("MSG", s, len(g), len(w), [x for x in g if x not in w][:2], [x for x in w if x not in g][:2]))
-        else:
-            for a, b in zip(got[s], want[s]):
-                if np.float32(a.level).view(np.uint32) != np.float32(b.level).view(np.uint32) or \
-                        np.float32(a.ppm).view(np.uint32) != np.float32(b.ppm).view(np.uint32):
-                    problems.append(("TAG", s, a.level, b.level, a.ppm, b.ppm))
     eng.close()
+    # messages (key, start/end idx) and tags (level, ppm bit patterns) in order, per stream
+    problems = [("MSG", s, len(got[s]), want[s][0]) for s in range(B) if G.msgs_digest(got[s]) != want[s]]
     assert not problems, "parity problems (first 12): %r" % (problems[:12],)
-    return n
+    return sum(w[0] for w in want)
 
 
 @pytest.mark.parametrize("fs,N", [(1536000, 65536), (1536000, 16384), (1536000, 4096), (384000, 16384), (3072000, 131072)])
@@ -386,16 +369,16 @@ def test_challenger(built, fs, N):
 def test_challenger_dense(built):
     # many overlapping / back-to-back bursts: frames complete in both branches close together, the Reset crosses branches
     xs = [S.fuzz_stream(96000, 262144, 300 + s)[0] for s in range(6)]
+    want = G.reference("challenger_dense", lambda: [G.msgs_digest(O.RefModel(model=O.MODEL_CHALLENGER, sample_rate=96000).run(x, 8192).messages())
+                                                    for x in xs])
     eng = aisgpu.Engine(model=aisgpu.MODEL_CHALLENGER, sample_rate=96000, n_streams=6, max_chunk=8192)
     got = [[] for _ in range(6)]
     for c in range(32):
         eng.submit(np.stack([x[c * 8192:(c + 1) * 8192] for x in xs]), 8192)
     for m in eng.poll():
-        got[m.stream].append((m.key(), m.start_idx, m.end_idx))
+        got[m.stream].append(m)
     for s in range(6):
-        r = O.RefModel(model=O.MODEL_CHALLENGER, sample_rate=96000)
-        r.run(xs[s], 8192)
-        assert got[s] == [(m.key(), m.start_idx, m.end_idx) for m in r.messages()], "stream %d" % s
+        assert G.msgs_digest(got[s]) == want[s], "stream %d" % s
     eng.close()
 
 
